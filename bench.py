@@ -2,7 +2,7 @@
 """bench.py — BASELINE.json metric: EKF-SLAM frames/sec @320x240, N = 100 features (config C4:
 n = 313, m = 200, 11x11 patch, +-20 px search ellipse), aggregate over independent camera streams.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams B] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams B] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one GoOneStep pass (predict -> select -> patch search -> EKF update -> normalise ->
 cull -> symmetrise) of every camera stream resident on the GPU over one new frame each.
@@ -12,6 +12,8 @@ cull -> symmetrise) of every camera stream resident on the GPU over one new fram
 Multi-GPU: replicas only (independent camera sequences, no collective on the data path); the
 barrier + max-over-ranks timing uses torch.distributed (NCCL).
 `--impl reference`: the CPU oracle (a port: the reference cannot be built here) on all host cores.
+`--dump-outputs DIR`: after the timed steps of the main workload, what they computed (see dump_outputs) as
+           DIR/<name>.npy, so that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -51,6 +53,8 @@ def parse():
     ap.add_argument("--only-main", action="store_true", help="skip the legs of the other configs / single stream")
     ap.add_argument("--step-groups", type=int, default=1, choices=[1, 2],
                     help="staggered stream groups of the fused step (1 = serial kernel order)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the states / feature results of the last timed step as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -210,8 +214,6 @@ def run_reference(args, rank, world):
         last = cpu_run(scenes, budget, threads)
         if k >= args.warmup:
             vals.append(last["fps"])
-        if len(vals) >= 3 and time.time() - T0 > 240:
-            break
     v = float(np.mean(vals))
     sample = "%d streams (1 per pinned thread) x ~%.0f s of oracle steps per bench step" % (threads, budget)
     ref_src = reference_sources_rate(args.config)
@@ -253,7 +255,38 @@ def _traffic(config, kernel, B):
         return None
 
 
-def measure_config(args, config, B, steps, warmup, rank, local_rank, world, stream, dev, e2e=True, clocks=False):
+DUMP_COV_STREAMS = 16
+
+
+def dump_outputs(ctx, B, directory):
+    """What a caller of the step receives for every stream -- state x, covariance diagonal, per-feature results --
+    padded with NaN to the largest state / feature count, and the full covariance of a fixed, seeded sample of
+    DUMP_COV_STREAMS streams (all of them would exceed 64 MB at the C4 size).  float64 throughout."""
+    os.makedirs(directory, exist_ok=True)
+    nf = np.array([ctx.num_features(s) for s in range(B)])
+    n = 13 + 3 * int(nf.max())
+    N = int(nf.max())
+    pick = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_COV_STREAMS), replace=False))
+    out = {"num_features": nf.astype(np.float64), "state_x": np.full((B, n), np.nan),
+           "state_cov_diag": np.full((B, n), np.nan), "state_cov_streams": pick.astype(np.float64),
+           "state_cov": np.full((len(pick), n, n), np.nan)}
+    widths = {"h": 2, "z": 2, "S": 4, "flags": 1, "attempted": 1, "successful": 1, "select_rank": 1}
+    for k, w in widths.items():
+        out["feature_" + k] = np.full((B, N, w), np.nan)
+    for s in range(B):
+        x, P = ctx.get_state(s)
+        out["state_x"][s, :len(x)] = x
+        out["state_cov_diag"][s, :len(x)] = np.diag(P)
+        if s in pick:
+            out["state_cov"][np.searchsorted(pick, s), :len(x), :len(x)] = P
+        for k, v in ctx.features(s).items():
+            out["feature_" + k][s, :len(v)] = np.asarray(v, np.float64).reshape(len(v), widths[k])
+    for k, v in out.items():
+        np.save(os.path.join(directory, k + ".npy"), v)
+
+
+def measure_config(args, config, B, steps, warmup, rank, local_rank, world, stream, dev, e2e=True, clocks=False,
+                   dump=None):
     """One workload (BASELINE config) on this rank's GPU: device-resident throughput, end-to-end throughput through
     the C ABI with host frames, per-kernel times.  Returns a dict (times already MAX-reduced over ranks)."""
     import torch
@@ -320,6 +353,8 @@ def measure_config(args, config, B, steps, warmup, rank, local_rank, world, stre
         out["clocks"] = sampler.summary()
     out["ms_per_step"] = ms / steps
     out["value"] = world * B * steps / (ms * 1e-3)
+    if dump:
+        dump_outputs(ctx, B, dump)
 
     # ---- per-kernel durations (CUDA events on the launching stream, one sync per step) ----------
     ctx.enable_timing(True)
@@ -542,7 +577,7 @@ def run_ours(args, rank, local_rank, world):
 
     B = args.streams
     main, scenes = measure_config(args, args.config, B, args.steps, args.warmup, rank, local_rank, world, stream, dev,
-                                  clocks=True)
+                                  clocks=True, dump=args.dump_outputs if rank == 0 else None)
     # the other BASELINE configs (north star: N in {20, 50, 100}; C3 on 8 GPUs = C5) and the single-stream latency
     extra = {}
     if not args.only_main:
@@ -598,8 +633,6 @@ def run_ours(args, rank, local_rank, world):
         dist.destroy_process_group()
 
 
-T0 = time.time()
-
 if __name__ == "__main__":
     a = parse()
     rank = int(os.environ.get("RANK", "0"))
@@ -608,6 +641,8 @@ if __name__ == "__main__":
     if a.dist_selftest:
         dist_selftest(rank, world)
     elif a.impl == "reference":
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of --impl ours")
         run_reference(a, rank, world)
     else:
         run_ours(a, rank, local_rank, world)

@@ -14,6 +14,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = os.path.join(_HERE, "liboracle.so")
 _REF = os.path.join(_HERE, "_ref", "libsl2ref.so")
+SCENELIB2_SRC_FILE = os.path.join(_HERE, "_ref", "scenelib2_src")   # the SceneLib2 tree _ref was built from
 
 u8p = C.POINTER(C.c_uint8)
 i32p = C.POINTER(C.c_int32)
@@ -38,7 +39,7 @@ def build(force=False):
     """Compile liboracle.so (and _ref when /root/reference exists).  Building is not using."""
     have_ref = os.path.isdir("/root/reference/scenelib2/improc")
     refm = os.path.join(_HERE, "_ref", "libsl2refmodels.so")
-    libs = [_LIB] + ([_REF, refm] if have_ref else [])
+    libs = [_LIB] + ([_REF, refm, SCENELIB2_SRC_FILE] if have_ref else [])
     stale = force or any(not os.path.exists(p) for p in libs)
     if not stale:
         newest_src = 0.0
@@ -90,6 +91,14 @@ def lib():
             getattr(L, name).restype = None
         _lib = L
     return _lib
+
+
+def scenelib2_src():
+    """The SceneLib2 source tree oracle/_ref was built from, or None when _ref was not built here."""
+    if not os.path.exists(SCENELIB2_SRC_FILE):
+        return None
+    d = open(SCENELIB2_SRC_FILE).read().strip()
+    return d if os.path.isdir(d) else None
 
 
 def ref():

@@ -19,12 +19,13 @@ def oracle():
     return pyoracle
 
 
-@pytest.fixture(scope="session")
-def refimpl(oracle):
-    r = oracle.ref()
-    if r is None:
-        pytest.skip("oracle/_ref/libsl2ref.so not built (reference tree absent)")
-    return r
+@pytest.fixture
+def ref(request, oracle):
+    """Outputs of the original SceneLib2 sources for this test (tests/refgolden.py)."""
+    from refgolden import Recording
+    r = Recording(request.node.name[len("test_"):], oracle)
+    yield r
+    r.close()
 
 
 @pytest.fixture(scope="session")

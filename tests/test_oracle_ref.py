@@ -1,11 +1,14 @@
-"""Pins the oracle's patch-correlation restatement (A1, A11, and through A11 the A2 loop) to the
-REFERENCE's own source: golden vectors under tests/golden/ were produced by
-oracle/_ref/libsl2ref.so = /root/reference/scenelib2/improc/{improc,search_multiple_overlapping_
-ellipses}.cpp compiled unmodified (see tests/golden/make_golden.py).  Bit-exact."""
+"""Pins the oracle's patch-correlation restatement (A1, A11, and through A11 the A2 loop), its models and its
+whole tracking step to the REFERENCE's own source: SceneLib2's improc/{improc,search_multiple_overlapping_ellipses}.cpp
+compiled unmodified (oracle/_ref/libsl2ref.so, golden vectors of tests/golden/make_golden.py; bit-exact) and its
+tracking core compiled against oracle/stubs_arith (oracle/_ref/libsl2refmodels.so).  The outputs of that code for
+the inputs below are stored under tests/golden/ref_*.npz (the `ref` fixture, tests/refgolden.py)."""
 import os
 
 import numpy as np
 import pytest
+
+from refgolden import assert_cov_close, cov_sample, digest, pick
 
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -29,7 +32,7 @@ def test_a11_matches_reference_golden(oracle):
     assert rf.any() and not rf.all()
 
 
-def test_a1_live_reference_random(oracle, refimpl):
+def test_a1_live_reference_random(oracle, ref):
     rng = np.random.default_rng(7)
     for B in (11, 15, 9):
         img = rng.integers(0, 256, (40, 50), dtype=np.uint8)
@@ -37,11 +40,11 @@ def test_a1_live_reference_random(oracle, refimpl):
             patch = rng.integers(0, 256, (B, B), dtype=np.uint8)
             x1, y1 = int(rng.integers(0, 50 - B)), int(rng.integers(0, 40 - B))
             a = oracle.correlate2_warning(patch, img, x1, y1)
-            b = oracle.correlate2_warning(patch, img, x1, y1, use_ref=True)
+            b = ref.take("a1", lambda: oracle.correlate2_warning(patch, img, x1, y1, use_ref=True))
             assert np.array(a).tobytes() == np.array(b).tobytes()
 
 
-def test_a11_live_reference_random(oracle, refimpl):
+def test_a11_live_reference_random(oracle, ref):
     from scenelib2_b200 import synth
     rng = np.random.default_rng(11)
     img = synth.make_texture(rng, 96, 128)
@@ -59,7 +62,7 @@ def test_a11_live_reference_random(oracle, refimpl):
             pu.append([Si[0, 0], Si[0, 1], Si[1, 1]])
         pu = np.array(pu)
         a = oracle.smoe_search(img, patch, pu, centres)
-        b = oracle.smoe_search(img, patch, pu, centres, use_ref=True)
+        b = ref.take("a11", lambda: oracle.smoe_search(img, patch, pu, centres, use_ref=True))
         for x, y in zip(a[:3], b[:3]):
             assert (x == y).all()
 
@@ -101,7 +104,7 @@ def _random_xv(rng, normalise=True):
     return xv
 
 
-def test_motion_model_matches_reference_source(oracle, refmodels):
+def test_motion_model_matches_reference_source(oracle, ref):
     rng = np.random.default_rng(31)
     worst = 0.0
     for k in range(200):
@@ -111,18 +114,19 @@ def test_motion_model_matches_reference_source(oracle, refmodels):
         dt = [1 / 30.0, 0.05, 0.01][k % 3]
         u = rng.normal(0, 1, 3) if k % 4 == 0 else np.zeros(3)
         a = oracle.motion(xv, dt, u)
-        b = oracle.motion(xv, dt, u, use_ref=True)
+        b = ref.take("motion", lambda: [pick(v, k, 16) for v in oracle.motion(xv, dt, u, use_ref=True)])
         for x, y in zip(a, b):
+            x = pick(x, k, 16)
             assert np.isfinite(y).all()
             worst = max(worst, np.abs(x - y).max() / max(1.0, np.abs(y).max()))
         J = oracle.dxvnorm_by_dxv(xv)
-        Jr, xn = oracle.dxvnorm_by_dxv(xv, use_ref=True)
-        assert (J == Jr).all()                               # scalar formulas only: bit-exact
-        assert (xn == xv).all()                              # quirk Q1: xv comes back un-normalised
+        Jr, xn = ref.take("dxvnorm", lambda: [digest(v) for v in oracle.dxvnorm_by_dxv(xv, use_ref=True)])
+        assert (digest(J) == Jr).all()                       # scalar formulas only: bit-exact
+        assert (digest(xv) == xn).all()                      # quirk Q1: xv comes back un-normalised
     assert worst < 1e-15, worst
 
 
-def test_measurement_model_matches_reference_source(oracle, refmodels):
+def test_measurement_model_matches_reference_source(oracle, ref):
     rng = np.random.default_rng(32)
     cams = [np.array([320, 240, 195.0, 195.0, 162.0, 125.0, 9e-6, 1.0]),
             np.array([640, 480, 390.0, 392.0, 322.0, 247.0, 2e-6, 2.0])]
@@ -140,8 +144,10 @@ def test_measurement_model_matches_reference_source(oracle, refmodels):
         P = A @ A.T * 1e-4 + 1e-6 * np.eye(16)
         Pxx, Pxy, Pyy = P[:13, :13], P[:13, 13:], P[13:, 13:]
         a = oracle.predict_feature(cam8, xv, y, Pxx, Pxy, Pyy)
-        b = oracle.predict_feature(cam8, xv, y, Pxx, Pxy, Pyy, use_ref=True)
+        b = ref.take("predict", lambda: [pick(v, k, 4) for v in
+                                         oracle.predict_feature(cam8, xv, y, Pxx, Pxy, Pyy, use_ref=True)])
         for x, r in zip(a, b):
+            x = pick(x, k, 4)
             if np.isfinite(r).all():
                 worst = max(worst, np.abs(x - r).max() / max(1.0, np.abs(r).max()))
             else:
@@ -151,14 +157,14 @@ def test_measurement_model_matches_reference_source(oracle, refmodels):
         xp_org[3:7] = [1, 0, 0, 0] + rng.normal(0, 0.3, 4)
         h = a[0] if np.isfinite(a[0]).all() else np.array([100.0, 100.0])
         va = oracle.visibility_test(cam8, xv[:7], y, xp_org, h)
-        vb = oracle.visibility_test(cam8, xv[:7], y, xp_org, h, use_ref=True)
+        vb = ref.take("visibility", lambda: oracle.visibility_test(cam8, xv[:7], y, xp_org, h, use_ref=True))
         assert va == vb, (k, va, vb)
         flags_seen.add(vb)
     assert worst < 1e-13, worst
     assert 0 in flags_seen and len(flags_seen) >= 5          # visible and several distinct failure codes
 
 
-def test_particle_prediction_matches_reference_source(oracle, refmodels):
+def test_particle_prediction_matches_reference_source(oracle, ref):
     """N2 prediction (monoslam.cpp:1347-1400): the oracle's PartFeatureModel::predict_particle against the
     reference's own part_feature_model.cpp / feature_model.cpp / feature_init_info.cpp (compiled unmodified
     against oracle/stubs_arith): h, S, S^-1, det S per depth particle."""
@@ -177,14 +183,16 @@ def test_particle_prediction_matches_reference_source(oracle, refmodels):
         P = A @ A.T * 1e-4 + 1e-6 * np.eye(19)
         lam = np.sort(rng.uniform(0.3, 6.0, 9))
         a = oracle.predict_particles(cam8, xv, ypi, lam, P[:13, :13], P[:13, 13:], P[13:, 13:])
-        b = oracle.predict_particles(cam8, xv, ypi, lam, P[:13, :13], P[:13, 13:], P[13:, 13:], use_ref=True)
+        b = ref.take("particles", lambda: [pick(v, k, 4) for v in oracle.predict_particles(
+            cam8, xv, ypi, lam, P[:13, :13], P[:13, 13:], P[13:, 13:], use_ref=True)])
         for x, r in zip(a, b):
+            x = pick(x, k, 4)
             assert np.isfinite(r).all()
             worst = max(worst, np.abs(x - r).max() / max(1.0, np.abs(r).max()))
     assert worst < 1e-13, worst
 
 
-def test_sinv_matches_reference_source(oracle, refmodels):
+def test_sinv_matches_reference_source(oracle, ref):
     """Particle::set_S (the reference's own feature_init_info.cpp:55-63, compiled against oracle/stubs_arith)
     runs the same LLT -> matrixL -> inverse -> L^-T L^-1 sequence as MonoSLAM::measure_feature
     (monoslam.cpp:371-374), i.e. the oracle's S -> PuInv (A3).  (The particle bookkeeping of that file is
@@ -194,7 +202,7 @@ def test_sinv_matches_reference_source(oracle, refmodels):
         a, b = rng.uniform(1, 400, 2)
         r = rng.uniform(-0.95, 0.95)
         S = np.array([[a, r * np.sqrt(a * b)], [r * np.sqrt(a * b), b]])
-        Sinv_ref, det_ref = oracle.particle_set_S_ref(S)
+        Sinv_ref, det_ref = ref.take("set_S", lambda: oracle.particle_set_S_ref(S))
         pu = oracle.puinv_from_S(S)
         ref3 = np.array([Sinv_ref[0, 0], Sinv_ref[0, 1], Sinv_ref[1, 1]])
         np.testing.assert_allclose(pu, ref3, rtol=4e-15, atol=0)
@@ -207,9 +215,27 @@ def test_sinv_matches_reference_source(oracle, refmodels):
 # fill_* / GoOneStep (oracle/ref_slam_shim.cpp), vs the oracle.  Integer results must be identical; state and
 # covariance agree up to summation order (the stand-in matrix class is not Eigen).
 
-def _compare_step(r, o, t, tol):
-    fr, fo = r.features(), o.features()
-    assert r.num_features == o.num_features and r.n == o.n
+def ref_state(r):
+    """What the comparisons use of the reference's state: x, and a cov_sample of P (keys P_*)."""
+    x, P = r.get_state()
+    return dict(x=x, num_features=r.num_features, n=r.n, **{"P_" + k: v for k, v in cov_sample(P).items()})
+
+
+def ref_step(ref, key, r, frame):
+    """One GoOneStep of the reference slam `r` (recording only) -> its features and ref_state."""
+    def run():
+        r.step(frame)
+        return dict(r.features(), **ref_state(r))
+    return ref.take(key, run)
+
+
+def ref_cov(fr):
+    return {k[2:]: v for k, v in fr.items() if k.startswith("P_")}
+
+
+def _compare_step(fr, o, t, tol):
+    fo = o.features()
+    assert fr["num_features"] == o.num_features and fr["n"] == o.n
     assert (fr["label"] == fo["label"]).all()
     assert (fr["select_rank"] == fo["select_rank"]).all(), t
     assert ((fr["flags"] & 1) == (fo["flags"] & 1)).all(), t
@@ -221,39 +247,41 @@ def _compare_step(r, o, t, tol):
     sel = fo["select_rank"] >= 0
     np.testing.assert_allclose(fr["h"][sel], fo["h"][sel], rtol=tol, atol=tol)
     np.testing.assert_allclose(fr["S"][sel], fo["S"][sel], rtol=tol, atol=tol)
-    xr, Pr = r.get_state()
     xo, Po = o.get_state()
     d = np.sqrt(np.abs(np.diag(Po))) + 1e-300
-    assert np.abs(xr - xo).max() <= tol * max(1.0, np.abs(xo).max())
-    assert (np.abs(Pr - Po) <= tol * d[:, None] * d[None, :]).all()
-    assert np.abs(Pr - Pr.T).max() == 0.0
+    assert np.abs(fr["x"] - xo).max() <= tol * max(1.0, np.abs(xo).max())
+    assert_cov_close(Po, ref_cov(fr), tol, d)
+    assert fr["P_asym"] == 0.0
 
 
-def test_whole_step_matches_reference_source(oracle, refmodels, tmp_path):
+def test_whole_step_matches_reference_source(oracle, ref, tmp_path):
     from scenelib2_b200 import synth
     from test_oracle_slam import make_oracle_slam
     kp = np.load(os.path.join(G, "known_patches.npy"))
     # C1: 20 features, 10 selected per frame by trace(S), ellipses from the EKF's own S_i
     sc = synth.make_scene("C1", n_frames=12, known_patches=kp)
-    r, o = oracle.RefSlam(sc, str(tmp_path / "c1")), make_oracle_slam(oracle, sc)
-    xr, Pr = r.get_state()
+    r = oracle.RefSlam(sc, str(tmp_path / "c1")) if ref.recording else None
+    o = make_oracle_slam(oracle, sc)
+    fr = ref.take("c1_init", lambda: ref_state(r))
     xo, Po = o.get_state()
-    assert (xr == xo).all() and (Pr == Po).all()          # Init + AddNewKnownFeature + fill_* round trip
+    assert (fr["x"] == xo).all()                          # Init + AddNewKnownFeature + fill_* round trip
+    assert_cov_close(Po, ref_cov(fr), 0.0, np.ones(len(xo)))
     for t in range(12):
-        r.step(sc.frames[t])
+        fr = ref_step(ref, "c1", r, sc.frames[t])
         o.step(sc.frames[t])
-        _compare_step(r, o, t, 1e-12)
+        _compare_step(fr, o, t, 1e-12)
     # C2-like without the benchmark's ellipse override: every feature selected (m = 2N), bigger update
     sc = synth.make_scene("C2", n_frames=4, n_features=24, override=False)
-    r, o = oracle.RefSlam(sc, str(tmp_path / "c2")), make_oracle_slam(oracle, sc)
+    r = oracle.RefSlam(sc, str(tmp_path / "c2")) if ref.recording else None
+    o = make_oracle_slam(oracle, sc)
     for t in range(4):
-        r.step(sc.frames[t])
+        fr = ref_step(ref, "c2", r, sc.frames[t])
         o.step(sc.frames[t])
-        _compare_step(r, o, t, 1e-11)
+        _compare_step(fr, o, t, 1e-11)
     assert (o.features()["select_rank"] >= 0).sum() == 24
 
 
-def test_bad_feature_deletion_matches_reference_source(oracle, refmodels, tmp_path):
+def test_bad_feature_deletion_matches_reference_source(oracle, ref, tmp_path):
     """delete_bad_features / delete_feature (monoslam.cpp:644-703, 770-812): a template that never matches is
     culled after 10 attempts; the compaction of state, covariance blocks and lists is the reference's own."""
     from scenelib2_b200 import synth
@@ -262,13 +290,14 @@ def test_bad_feature_deletion_matches_reference_source(oracle, refmodels, tmp_pa
     bad = sc.patches.copy()
     bad[3] = np.random.default_rng(0).integers(0, 256, bad[3].shape, dtype=np.uint8)
     sc.patches = bad
-    r, o = oracle.RefSlam(sc, str(tmp_path)), make_oracle_slam(oracle, sc)
+    r = oracle.RefSlam(sc, str(tmp_path)) if ref.recording else None
+    o = make_oracle_slam(oracle, sc)
     n0 = o.n
     for t in range(12):
-        r.step(sc.frames[t % 2])
+        fr = ref_step(ref, "step", r, sc.frames[t % 2])
         o.step(sc.frames[t % 2])
-        _compare_step(r, o, t, 1e-11)
-    assert r.num_features == 11 and r.n == n0 - 3
+        _compare_step(fr, o, t, 1e-11)
+    assert fr["num_features"] == 11 and fr["n"] == n0 - 3
 
 
 def test_c1_trajectory_1000_steps_reproduced_by_reference_source(oracle, refmodels, tmp_path):
@@ -302,7 +331,7 @@ def test_c1_trajectory_1000_steps_reproduced_by_reference_source(oracle, refmode
     assert (f["attempted"] == k["attempted"]).all() and (f["successful"] == k["successful"]).all()
 
 
-def test_elliptical_search_and_detector_match_reference_source(oracle, refmodels):
+def test_elliptical_search_and_detector_match_reference_source(oracle, ref):
     """A2 / A3 / N3 one by one against the reference's own monoslam.cpp: MonoSLAM::elliptical_search (rotated and
     border-clamped ellipses, plateaus, 11x11 and 15x15), measure_feature (S -> PuInv -> search) and
     find_best_patch_inside_region (positions and FP64 eigenvalue bits)."""
@@ -326,7 +355,7 @@ def test_elliptical_search_and_detector_match_reference_source(oracle, refmodels
             centre = np.array([cu + rng.uniform(-4, 4), cv + rng.uniform(-4, 4)])
             if k % 7 == 0:
                 centre = np.array([rng.choice([1.5, 158.2]), rng.choice([2.4, 117.9])])   # clamped at a corner
-            ok, ru, rv = oracle.elliptical_search_ref(img, patch, centre, pu)
+            ok, ru, rv = ref.take("search", lambda: oracle.elliptical_search_ref(img, patch, centre, pu))
             ou, ov, of, _ = oracle.elliptical_search(img, patch[None], centre[None], pu[None])
             assert bool(of[0]) == bool(ok), (B, k)
             if ok:
@@ -340,7 +369,7 @@ def test_elliptical_search_and_detector_match_reference_source(oracle, refmodels
         r = rng.uniform(-0.8, 0.8)
         S = np.array([[a, r * np.sqrt(a * b)], [r * np.sqrt(a * b), b]])
         hh = np.array([cu + rng.uniform(-3, 3), cv + rng.uniform(-3, 3)])
-        ok, z = oracle.measure_feature_ref(img, patch, hh, S)
+        ok, z = ref.take("measure", lambda: oracle.measure_feature_ref(img, patch, hh, S))
         pu = oracle.puinv_from_S(S)
         ou, ov, of, _ = oracle.elliptical_search(img, patch[None], hh[None], pu[None])
         assert bool(of[0]) == bool(ok), k
@@ -351,11 +380,11 @@ def test_elliptical_search_and_detector_match_reference_source(oracle, refmodels
     for B in (11, 15):
         for reg in regions:
             a = oracle.find_best_patch(img, B, reg, ubest=-7, vbest=-9)
-            b = oracle.find_best_patch(img, B, reg, ubest=-7, vbest=-9, use_ref=True)
+            b = ref.take("best_patch", lambda: oracle.find_best_patch(img, B, reg, ubest=-7, vbest=-9, use_ref=True))
             assert a[:2] == b[:2] and np.float64(a[2]).tobytes() == np.float64(b[2]).tobytes(), (B, reg)
 
 
-def test_particle_cycle_matches_reference_source(oracle, refmodels, tmp_path):
+def test_particle_cycle_matches_reference_source(oracle, ref, tmp_path):
     """N2 end to end on the reference's own code: InitialiseFeature creates a partially-initialised feature with
     100 depth particles; after the camera has moved, predict_partially_initialised_feature_measurements
     (part_feature_model.cpp), measure_feature_with_multiple_priors (SMOE) and
@@ -367,16 +396,23 @@ def test_particle_cycle_matches_reference_source(oracle, refmodels, tmp_path):
     sc = synth.make_scene("C1", n_frames=6, known_patches=kp)
     cycles = 0
     for (u, v, dx) in ((150, 110, (0.03, -0.01, 0.0)), (90, 70, (-0.02, 0.02, 0.01)), (200, 150, (0.0, 0.04, 0.0))):
-        r = oracle.RefSlam(sc, str(tmp_path / ("p%d_%d" % (u, v))))
-        r.init_partial_feature(sc.frames[0], u, v)
-        assert r.num_features == sc.n_features + 1 and r.n == 13 + 3 * sc.n_features + 6
-        assert r.particle_cycle(sc.frames[0]) is None          # no match attempt right after initialisation
+        r = oracle.RefSlam(sc, str(tmp_path / ("p%d_%d" % (u, v)))) if ref.recording else None
+
+        def init():
+            r.init_partial_feature(sc.frames[0], u, v)
+            return r.num_features, r.n
+        nf, n = ref.take("init", init)
+        assert nf == sc.n_features + 1 and n == 13 + 3 * sc.n_features + 6
+        # no match attempt right after initialisation
+        assert ref.take("cycle", lambda: r.particle_cycle(sc.frames[0])) is None
         patch = sc.frames[0][v - 5:v + 6, u - 5:u + 6]
         for t in (1, 2, 3):
-            x, P = r.get_state()
-            x[:3] += dx                                        # the camera moves: the depth line spreads out
-            r.set_state(x, P)
-            c = r.particle_cycle(sc.frames[t])
+            def cycle():
+                x, P = r.get_state()
+                x[:3] += dx                                    # the camera moves: the depth line spreads out
+                r.set_state(x, P)
+                return r.particle_cycle(sc.frames[t])
+            c = ref.take("cycle", cycle)
             if c is None:
                 break
             ou, ov, of, _ = oracle.smoe_search(sc.frames[t], patch, c["sinv3"], c["h"])
@@ -395,17 +431,18 @@ def test_particle_cycle_matches_reference_source(oracle, refmodels, tmp_path):
     assert cycles >= 4
 
 
-def test_c4_size_step_matches_reference_source(oracle, refmodels, tmp_path):
+def test_c4_size_step_matches_reference_source(oracle, ref, tmp_path):
     """Full-size update (n = 313, all 100 features measured, m = 200; ellipses from the EKF's own S_i since the
     reference has no fixed-ellipse switch): Kalman::KalmanFilterUpdate as written (kalman.cpp:72-119) with its
     gather / scatter, on the reference's own code vs the oracle."""
     from scenelib2_b200 import synth
     from test_oracle_slam import make_oracle_slam
     sc = synth.make_scene("C4", n_frames=3, override=False)
-    r, o = oracle.RefSlam(sc, str(tmp_path)), make_oracle_slam(oracle, sc)
+    r = oracle.RefSlam(sc, str(tmp_path)) if ref.recording else None
+    o = make_oracle_slam(oracle, sc)
     for t in range(3):
-        r.step(sc.frames[t])
+        fr = ref_step(ref, "step", r, sc.frames[t])
         o.step(sc.frames[t])
-        _compare_step(r, o, t, 1e-11)
+        _compare_step(fr, o, t, 1e-11)
     f = o.features()
     assert ((f["flags"] & 2) > 0).sum() == 100 and o.n == 313
