@@ -60,6 +60,59 @@ def assert_state_close(xg, Pg, xo, Po, rtol=RTOL_TEST):
     return ex, eP
 
 
+def random_measurements(rng, n, nf, K):
+    """K distinct measured features of an nf-feature map (state size n): their rows of H (dense dh/dxv in the first 7
+    columns, dh/dy on the feature's 3 columns), isotropic R blocks and an innovation nu.  Returns the ABI's pieces
+    (feats, Hxv, Hy, R as K x 2 x 2) and the dense H and R of the same update."""
+    feats = rng.permutation(nf)[:K].astype(np.int32)
+    Hxv = np.zeros((2 * K, 13))
+    Hxv[:, :7] = rng.standard_normal((2 * K, 7)) * 60
+    Hy = rng.standard_normal((2 * K, 3)) * 300
+    var = rng.uniform(1, 4, K)
+    R = np.zeros((K, 2, 2))
+    R[:, 0, 0] = R[:, 1, 1] = var
+    nu = rng.standard_normal(2 * K) * 2
+    H = np.zeros((2 * K, n))
+    H[:, :13] = Hxv
+    for k, f in enumerate(feats):
+        H[2 * k:2 * k + 2, 13 + 3 * f:16 + 3 * f] = Hy[2 * k:2 * k + 2]
+    return feats, Hxv, Hy, R, nu, H, np.kron(np.diag(var), np.eye(2))
+
+
+def check_streams_against_oracle(ctx, oracles, picks, scenes_of, frame):
+    """Step the oracles of `picks` on `frame` and compare them with the context's streams after its step: map size,
+    selection, flags, match positions and counters exactly, state within RTOL_TEST, P exactly symmetric."""
+    for s in picks:
+        o = oracles[s]
+        o.step(scenes_of(s).frames[frame])
+        fg, fo = ctx.features(s), o.features()
+        assert ctx.num_features(s) == o.num_features, s
+        assert (fg["select_rank"] == fo["select_rank"]).all() and (fg["flags"] == fo["flags"]).all(), s
+        ok = (fo["flags"] & 2) > 0
+        assert (fg["z"][ok] == fo["z"][ok]).all(), s
+        assert (fg["attempted"] == fo["attempted"]).all() and (fg["successful"] == fo["successful"]).all(), s
+        xg, Pg = ctx.get_state(s)
+        assert_state_close(xg, Pg, *o.get_state())
+        assert np.abs(Pg - Pg.T).max() == 0.0
+
+
+def recipe_scene(cap, nf, n_bad, n_out, stream_id=0, n_frames=3):
+    """A C4 scene (fixed +-20 px search) with nf features that selects up to `cap` per frame, n_bad of them with a
+    template of noise (selected, never found) and n_out moved 3 m sideways (never visible, never selected): every
+    frame measures m = 2 (nf - n_bad - n_out) rows.  Which features are spoiled is drawn from a seeded permutation."""
+    sc = synth.make_scene("C4", stream_id=stream_id, n_frames=n_frames, n_features=nf)
+    sc.n_select = cap
+    rng = np.random.default_rng(1000 * cap + 7 * nf + stream_id)
+    perm = rng.permutation(nf)
+    sc.x0 = sc.x0.copy()
+    for i in perm[:n_out]:
+        sc.x0[13 + 3 * i] += 3.0
+    sc.patches = sc.patches.copy()
+    for i in perm[n_out:n_out + n_bad]:
+        sc.patches[i] = rng.integers(0, 256, sc.patches[i].shape, dtype=np.uint8)
+    return sc
+
+
 def random_puinv(rng, n, lo, hi, iso_fraction=0.5):
     out = np.zeros((n, 3))
     for i in range(n):

@@ -4,7 +4,7 @@ through the C ABI vs the CPU oracle.  Tolerance: the north star's 1e-5 relative,
 import numpy as np
 import pytest
 
-from gpu_util import (RTOL_TEST, assert_state_close, ctx_from_scenes, oracle_slam_from_scene,
+from gpu_util import (RTOL_TEST, assert_state_close, ctx_from_scenes, oracle_slam_from_scene, random_measurements,
                       state_err, synth)
 
 pytestmark = pytest.mark.gpu
@@ -41,22 +41,6 @@ def test_measurement_prediction_and_selection(oracle):
         ctx.close()
 
 
-def _random_measurements(rng, n, nf, K):
-    feats = rng.permutation(nf)[:K].astype(np.int32)
-    Hxv = np.zeros((2 * K, 13))
-    Hxv[:, :7] = rng.standard_normal((2 * K, 7)) * 60
-    Hy = rng.standard_normal((2 * K, 3)) * 300
-    var = rng.uniform(1, 4, K)
-    R = np.zeros((K, 2, 2))
-    R[:, 0, 0] = R[:, 1, 1] = var
-    nu = rng.standard_normal(2 * K) * 2
-    H = np.zeros((2 * K, n))
-    H[:, :13] = Hxv
-    for k, f in enumerate(feats):
-        H[2 * k:2 * k + 2, 13 + 3 * f:16 + 3 * f] = Hy[2 * k:2 * k + 2]
-    return feats, Hxv, Hy, R, nu, H, np.kron(np.diag(var), np.eye(2))
-
-
 @pytest.mark.parametrize("nf,K", [(20, 4), (20, 20), (50, 50), (100, 100), (37, 13), (128, 128), (128, 77),
                                   (5, 1), (9, 9)])
 def test_update_with_host_rows_matches_dense_oracle(oracle, nf, K):
@@ -65,7 +49,7 @@ def test_update_with_host_rows_matches_dense_oracle(oracle, nf, K):
     ctx = ctx_from_scenes([sc])
     rng = np.random.default_rng(nf * 1000 + K)
     n = sc.n
-    feats, Hxv, Hy, R, nu, H, Rfull = _random_measurements(rng, n, nf, K)
+    feats, Hxv, Hy, R, nu, H, Rfull = random_measurements(rng, n, nf, K)
     ctx.ekf_update(0, feats, Hxv, Hy, R, nu)
     xg, Pg = ctx.get_state(0)
     xo, Po = oracle.kalman_update_dense(sc.x0, sc.P0, H, Rfull, nu)
@@ -139,7 +123,7 @@ def test_update_honours_full_2x2_R_and_rejects_asymmetric(oracle):
     ctx = ctx_from_scenes([sc])
     rng = np.random.default_rng(77)
     n = sc.n
-    feats, Hxv, Hy, R, nu, H, _ = _random_measurements(rng, n, nf, K)
+    feats, Hxv, Hy, R, nu, H, _ = random_measurements(rng, n, nf, K)
     Hxv[:, 7:] = rng.standard_normal((2 * K, 6)) * 20      # all 13 dh/dxv columns, not only [dh/dxp | 0]
     H[:, :13] = Hxv
     for k in range(K):                                     # anisotropic, correlated measurement noise

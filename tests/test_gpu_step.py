@@ -5,8 +5,8 @@ import os
 import numpy as np
 import pytest
 
-from gpu_util import (RTOL_NORTH_STAR, RTOL_TEST, assert_state_close, ctx_from_scenes, oracle_slam_from_scene,
-                      sl2, state_err, synth)
+from gpu_util import (RTOL_NORTH_STAR, RTOL_TEST, assert_state_close, check_streams_against_oracle, ctx_from_scenes,
+                      oracle_slam_from_scene, sl2, state_err, synth)
 
 pytestmark = pytest.mark.gpu
 G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -354,21 +354,6 @@ def test_cuda_path_against_the_reference_source():
         ctx.close()
 
 
-def _check_streams_against_oracle(ctx, oracles, picks, scenes_of, frame):
-    for s in picks:
-        o = oracles[s]
-        o.step(scenes_of(s).frames[frame])
-        fg, fo = ctx.features(s), o.features()
-        assert ctx.num_features(s) == o.num_features, s
-        assert (fg["select_rank"] == fo["select_rank"]).all() and (fg["flags"] == fo["flags"]).all(), s
-        ok = (fo["flags"] & 2) > 0
-        assert (fg["z"][ok] == fo["z"][ok]).all(), s
-        assert (fg["attempted"] == fo["attempted"]).all() and (fg["successful"] == fo["successful"]).all(), s
-        xg, Pg = ctx.get_state(s)
-        assert_state_close(xg, Pg, *o.get_state())
-        assert np.abs(Pg - Pg.T).max() == 0.0
-
-
 def test_c4_bench_shape_296_streams_against_oracle(oracle):
     """The shape bench.py runs (BASELINE C4, 296 camera streams in one context: 2 per SM), 3 frames, with the first,
     the two middle and the last stream compared with the oracle -- a stream-indexing bug above the sizes of the other
@@ -384,7 +369,7 @@ def test_c4_bench_shape_296_streams_against_oracle(oracle):
         cfg_ctx.set_frames(t % 2, np.stack([scene_of(s).frames[t] for s in range(B)]))
         cfg_ctx.step(t % 2)
         cfg_ctx.sync()
-        _check_streams_against_oracle(cfg_ctx, oracles, picks, scene_of, t)
+        check_streams_against_oracle(cfg_ctx, oracles, picks, scene_of, t)
         for s in range(0, B, 7):
             sc = scene_of(s)
             f = cfg_ctx.features(s)
@@ -460,7 +445,7 @@ def test_c3_four_streams_four_frames_against_oracle(oracle):
         ctx.set_frames(t % 2, np.stack([sc.frames[t] for sc in scenes]))
         ctx.step(t % 2)
         ctx.sync()
-        _check_streams_against_oracle(ctx, oracles, range(B), lambda s: scenes[s], t)
+        check_streams_against_oracle(ctx, oracles, range(B), lambda s: scenes[s], t)
     ctx.close()
 
 

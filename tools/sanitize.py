@@ -1,10 +1,33 @@
-"""Small end-to-end exercise of every kernel for compute-sanitizer (memcheck / racecheck)."""
+"""Small end-to-end exercise of every kernel for compute-sanitizer (memcheck / racecheck).
+`python tools/sanitize.py update-shapes` runs only the batched EKF update launch shapes at the end."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np
 from scenelib2_b200 import synth
-from gpu_util import ctx_from_scenes, random_puinv
+from gpu_util import ctx_from_scenes, random_puinv, recipe_scene
+
+
+def update_shapes():
+    """One fused step per batched update shape of tests/test_gpu_update_shapes.py, 8 streams of different m and n per
+    context: upd_solve_kernel<10> (capacity 80) spread and batched; the walking solve at NP = 4 and 7 (148 streams);
+    the one-CTA plain upd_hp with two column chunks (capacity 104, 296 streams); a 296-stream two-group step."""
+    from test_gpu_update_shapes import BATCH_RECIPES
+    for cap, B, groups in ((80, 8, 1), (80, 296, 1), (32, 148, 1), (56, 148, 1), (104, 296, 1), (80, 296, 2)):
+        uniq = [recipe_scene(cap, *r, stream_id=i, n_frames=1) for i, r in enumerate(BATCH_RECIPES[cap])]
+        scs = [uniq[(5 * s) % 8] for s in range(B)]
+        c = ctx_from_scenes(scs, max_features=cap)
+        c.set_step_groups(groups)
+        c.set_frames(0, np.stack([sc_.frames[0] for sc_ in scs])); c.step(0); c.sync()
+        print("update shape cap=%d streams=%d groups=%d: map sizes %s, state finite: %s" % (
+            cap, B, groups, [c.num_features(s) for s in range(8)],
+            all(np.isfinite(c.get_state(s)[1]).all() for s in range(0, B, 37))))
+        c.close()
+
+
+if sys.argv[1:] == ["update-shapes"]:
+    update_shapes()
+    sys.exit(0)
 
 scenes = [synth.make_scene("C2", stream_id=s, n_frames=3, n_features=21, override=(s == 0)) for s in range(2)]
 ctx = ctx_from_scenes(scenes, frame_slots=2)
@@ -79,3 +102,4 @@ ca.append_feature(0, np.array([0.0, 0.1, 1.2]), scenes[0].xp_org[1], scenes[0].p
 print("big state finite:", bool(np.isfinite(cb.get_state(1)[1]).all()), "appended:", ca.num_features(0))
 print("found", int(f.sum()), "of", n, "| state finite:", bool(np.isfinite(ctx.get_state(0)[1]).all()),
       bool(np.isfinite(c3.get_state(0)[1]).all()))
+update_shapes()
